@@ -3,6 +3,7 @@
 "WaveNet train audio-samples/sec/GPU; Tacotron mel-frames/sec; 1/2/4/8 B200").
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME]      # our arm (CUDA, one process per GPU)
+  python bench.py [...] --dump-outputs DIR                                   # + one timed step from the seeded state, as DIR/*.npy
   python bench.py --impl reference [...]                                     # CPU arm: the oracle restatement of the reference
                                                                              # graph on the host cores (TF1 cannot be installed
                                                                              # here; DESIGN.md §2)
@@ -395,6 +396,39 @@ def make_workload(name):
     return TacotronWorkload() if name == "tacotron" else WaveNetWorkload(name)
 
 
+DUMP_SAMPLE = 1 << 22          # elements kept of a larger flat buffer: 3 buffers x 16 MB + the loss stay under 64 MB
+
+
+def restore_initial_state(model, params0):
+    """Puts a model back where setup() left it: the seeded variables, no Adam moments or EMA shadows yet, step counters at zero
+    (the dropout seed of the next step is then the first step's)."""
+    model.params.copy_(params0)
+    model.m = model.v = None
+    if hasattr(model, "ema"):
+        model.ema = None
+    model.global_step = 0
+    model.step_dev.zero_()
+    for flag in ("_packed_dirty", "_dirty"):        # the eager path re-packs the bf16 operand copies before its next forward
+        if hasattr(model, flag):
+            setattr(model, flag, True)
+
+
+def dump_outputs(model, out_dir):
+    """Writes what a training step hands its caller as float32 .npy files: the loss buffer, the gradients, the updated parameters
+    and (WaveNet) their EMA shadows. A flat buffer longer than DUMP_SAMPLE is written as a fixed, seeded sample of its elements in
+    index order, the same indices for every buffer of that length."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name in ("loss_buf", "grads", "params", "ema"):
+        t = getattr(model, name, None)
+        if t is None:
+            continue
+        a = t.detach().float().cpu().numpy()
+        if a.size > DUMP_SAMPLE:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ---------------------------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -405,7 +439,14 @@ def main():
     ap.add_argument("--workload", default="wavenet_ce", choices=["wavenet_ce", "wavenet_mol", "wavenet_default", "tacotron"])
     ap.add_argument("--no-graph", action="store_true", help="launch kernels eagerly instead of replaying a CUDA graph")
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the bounded oracle timing on rank 0")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, run the timed step once more from the seeded initial "
+                                                         "variables and write what it computed to DIR/<name>.npy (rank 0), so that "
+                                                         "runs with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     heavy = args.workload != "wavenet_ce"
     steps = args.steps if args.steps is not None else (20 if heavy else 200)
     warmup = args.warmup if args.warmup is not None else (3 if heavy else 10)
@@ -436,6 +477,7 @@ def main():
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
     wl.setup(dev, rank, not args.no_graph)
+    params0 = wl.model.params.clone() if args.dump_outputs else None
 
     def barrier():
         if world > 1:
@@ -467,6 +509,15 @@ def main():
     loss = wl.loss()
     ms_per_step = results["resident"] / steps
     roof = wl.roofline(ms_per_step)
+    if args.dump_outputs:
+        # The state after the timed steps is not reproducible: the kernels reduce with float atomics, and over many steps the bf16
+        # re-rounding of the weights and Adam on gradients that are zero up to rounding amplify that order noise far beyond
+        # rounding. One step of the timed call from the seeded variables and batch carries only that one step's order noise.
+        restore_initial_state(wl.model, params0)
+        wl.step(False, world)
+        barrier()
+        if rank == 0:
+            dump_outputs(wl.model, args.dump_outputs)
 
     if rank == 0:
         total_units = world * wl.units_per_gpu_step * steps

@@ -17,6 +17,7 @@ upsampling layers (`_init_kernel`, modules.py:642-654,761-770).
 
 Honesty: the layer primitives under the reference's code (tf.layers.Conv1D / Conv2D / Conv2DTranspose, keras Wrapper) are
 tf_shim_graph.py's restatement of the TF 1.x definitions; the reference's composition of them is executed unchanged."""
+import json
 import os
 import sys
 
@@ -44,6 +45,24 @@ SCENARIOS = {
     "gauss_paper_2d": dict(input_type="raw", quantize_channels=256, out_channels=2, upsample_type="2D", legacy=False, residual_legacy=False,
                            cdf_loss=True, log_scale_min_gauss=-7.000000006091266),
 }
+
+
+def save_packed(path, arrays):
+    """np.savez_compressed with the numeric arrays of each dtype concatenated into one entry `packed_<dtype>`, located through the
+    JSON list `packed_index` of (name, dtype, offset, shape): stored one by one, the ~1450 small arrays of this file would spend a
+    third of it on zip headers. tests/test_reference_wavenet_graph.py reads it back."""
+    index, groups, sizes, plain = [], {}, {}, {}
+    for name in sorted(arrays):
+        a = np.asarray(arrays[name])
+        if a.dtype.kind not in "biuf":
+            plain[name] = a
+            continue
+        key = a.dtype.name
+        index.append((name, key, sizes.get(key, 0), list(a.shape)))
+        groups.setdefault(key, []).append(a.reshape(-1))
+        sizes[key] = sizes.get(key, 0) + a.size
+    np.savez_compressed(path, packed_index=np.array(json.dumps(index)), **plain,
+                        **{"packed_" + k: np.concatenate(v) for k, v in groups.items()})
 
 
 def model_eval_loss(out, tag):
@@ -176,7 +195,7 @@ def main():
               out[tag + "_synth_y_hat"].shape))
 
     path = os.path.join(HERE, "reference_wavenet_graph.npz")
-    np.savez_compressed(path, **out)
+    save_packed(path, out)
     print("wrote %s: %d arrays, %.1f KB" % (path, len(out), os.path.getsize(path) / 1024))
 
 

@@ -53,7 +53,7 @@ def test_oracle_mulaw_float32_matches_reference_tensor_path():
     # for the record: numpy >= 2 promotes the reference's numpy float32 path to float64 at `/ np.log1p(255)`; that changes a
     # handful of indices that sit within one float32 ulp of a bin edge and nothing else
     d = R["mulaw_q_numpy_f32_numpy2"] != R["mulaw_q_tensor_f32"]
-    assert d[-40000:].mean() < 1e-4 and np.abs(R["mulaw_q_numpy_f32_numpy2"][d] - R["mulaw_q_tensor_f32"][d]).max(initial=0) <= 1
+    assert d[-2000:].mean() < 1e-4 and np.abs(R["mulaw_q_numpy_f32_numpy2"][d] - R["mulaw_q_tensor_f32"][d]).max(initial=0) <= 1
 
 
 @pytest.mark.gpu

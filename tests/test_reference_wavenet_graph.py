@@ -8,6 +8,7 @@ network output, the upsampled conditioning and the loss with the recorded dropou
 autograd through the executed reference graph; the NN_init kernels the reference's `_init_kernel` hands to its upsampling layers ==
 the oracle's and the product initialiser's."""
 import importlib
+import json
 import os
 
 import numpy as np
@@ -23,9 +24,25 @@ TAGS = ["ce_subpixel", "mol_2d", "gauss_nn", "gauss_paper_2d", "ce_resize", "ce_
 SUPPORTED = ["ce_subpixel", "mol_2d", "gauss_nn", "gauss_paper_2d"]          # configurations the CUDA path accepts; the rest is oracle only
 
 
+class _Arrays(dict):
+    """name -> array like np.load's NpzFile: `files` lists the names and every lookup returns a fresh copy"""
+    @property
+    def files(self):
+        return list(self)
+
+    def __getitem__(self, name):
+        return dict.__getitem__(self, name).copy()
+
+
 @pytest.fixture(scope="module")
 def R():
-    return np.load(PATH)
+    """the generator's save_packed() layout: numeric arrays concatenated per dtype, located through `packed_index`"""
+    z = np.load(PATH)
+    groups = {k: z[k] for k in z.files if k.startswith("packed_") and k != "packed_index"}
+    out = _Arrays((k, z[k]) for k in z.files if not k.startswith("packed_"))
+    for name, key, off, shape in json.loads(str(z["packed_index"])):
+        out[name] = groups["packed_" + key][off:off + int(np.prod(shape, dtype=np.int64))].reshape(shape)
+    return out
 
 
 def _hp(R, tag):
